@@ -2,11 +2,16 @@
 """bench.py -- SDF+grad queries/s of the batched signed-distance query path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload default|c4|c2|mesh10k|mesh50k|c3|c3cached|c5|c4readme]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
 
-One "step" = one pass of the hot path over one batch of synthetic input.
+One "step" = one pass of the hot path over one batch of synthetic input.  Every timed loop of a run times exactly K
+steps.
 
-DEFAULT (no --workload): the line the driver records.
+`--dump-outputs DIR` writes what the last timed step of the headline (or of the one --workload) returned, as
+DIR/value.npy and DIR/gradient.npy (rank 0).  Inputs are seeded, so two builds run with the same arguments can be
+compared output for output; see dump_outputs for the sampling of large results.
+
+DEFAULT (no --workload): the headline line.
   * headline = BASELINE.json configs[3] (C4), the workload north_star's multi-GPU target names: RobotSDF of a
     7-DOF arm (8 link SDFs), 200 joint configurations x 100 000 query points, value + gradient.  With N > 1
     (torchrun, one rank per GPU) the CONFIGURATION batch is split over the ranks (strong scaling: total work fixed)
@@ -30,8 +35,10 @@ wheels that are not installable in this image (SURVEY.md section 0), so the orac
 Prints ONE JSON line (rank 0).
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import statistics
 import sys
 import tempfile
@@ -52,6 +59,40 @@ OTHER_WORKLOADS = ("mesh10k", "c2", "c3", "c3cached", "c5")
 
 
 # ------------------------------------------------------------------------------------------------ helpers
+_scratch = None
+
+
+def scratch_dir():
+    """Directory for the files a run writes (link meshes, URDFs, SDF table caches): created fresh for this process,
+    so that no table cached by an earlier run or another build is read back, and removed when the process exits."""
+    global _scratch
+    if _scratch is None:
+        _scratch = tempfile.mkdtemp(prefix="pvb_bench_")
+        atexit.register(shutil.rmtree, _scratch, ignore_errors=True)
+    return _scratch
+
+
+DUMP_MAX_BYTES = 48 << 20
+
+
+def dump_outputs(out, dirname):
+    """Writes the tensors one step returned as <dirname>/value.npy [and gradient.npy], float32 (float64 kept).
+    Value is [..., P] and gradient [..., P, 3] over P query points; when they hold more than DUMP_MAX_BYTES, the
+    same seeded, sorted sample of the P points is kept in every run."""
+    tensors = [t for t in (out if isinstance(out, (tuple, list)) else (out,)) if torch.is_tensor(t)]
+    n = tensors[0].shape[-1]
+    per_point = sum(t.numel() // n * 4 * (2 if t.dtype == torch.float64 else 1) for t in tensors)
+    k = min(n, DUMP_MAX_BYTES // per_point)
+    idx = None if k == n else torch.randperm(n, generator=torch.Generator().manual_seed(0))[:k].sort().values
+    os.makedirs(dirname, exist_ok=True)
+    for name, t, axis in zip(("value", "gradient"), tensors, (-1, -2)):
+        if idx is not None:
+            t = t.index_select(t.dim() + axis, idx.to(t.device))
+        if t.dtype != torch.float64:
+            t = t.float()
+        np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy())
+
+
 def measured_peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
@@ -205,7 +246,7 @@ class C2(Workload):
         v, f = workloads.fixture_mesh("drill")
         self.obj = pv.MeshObjectFactory("drill", mesh=(v, f))
         gt = pv.MeshSDF(self.obj)
-        cache = os.path.join(cache_dir or tempfile.gettempdir(), f"pvb_bench_c2_{rank}.pkl")
+        cache = os.path.join(cache_dir or scratch_dir(), f"pvb_bench_c2_{rank}.pkl")
         self.sdf = pv.CachedSDF("drill", 0.005, self.obj.bounding_box(padding=0.1), gt, device="cuda",
                                 cache_path=cache, clean_cache=True)
         # same object for host callers: results come back as host tensors (tables still live on the GPU)
@@ -325,7 +366,7 @@ class C4(Workload):
         self.mode = mode if world > 1 else "none"
         self.peer = None
         self.peer_error = None
-        d = os.path.join(cache_dir or tempfile.gettempdir(), f"pvb_bench_arm_{rank}")
+        d = os.path.join(cache_dir or scratch_dir(), f"pvb_bench_arm_{rank}")
         urdf, end = workloads.write_arm(d)
         chain = pv.build_serial_chain_from_urdf(open(urdf).read(), end).to(device="cuda")
         self.robot = pv.RobotSDF(chain, path_prefix=d,
@@ -460,7 +501,7 @@ class C3(Workload):
         gt = pv.MeshSDF(obj)
         if cached:
             sub = pv.CachedSDF("drill", 0.005, obj.bounding_box(padding=0.1), gt, device="cuda",
-                               cache_path=os.path.join(cache_dir or tempfile.gettempdir(), f"pvb_c3_{rank}.pkl"))
+                               cache_path=os.path.join(cache_dir or scratch_dir(), f"pvb_c3_{rank}.pkl"))
         else:
             sub = gt
         tm = workloads.random_rigid(16, seed=1, t_range=0.5).cuda()
@@ -564,7 +605,7 @@ def cpu_arm(name):
                       "(sdf.py:392-433 restated: per-SDF loop + argmin)",
                       f"C3 ComposedSDF of 16 drills ({'CachedSDF res=0.005' if name == 'c3cached' else 'MeshSDF'})")
     if name in ("c4", "c4readme"):
-        d = os.path.join(tempfile.gettempdir(), "pvb_bench_arm_cpu")
+        d = os.path.join(scratch_dir(), "pvb_bench_arm_cpu")
         urdf, end = workloads.write_arm(d)
         chain = opk.build_serial_chain_from_urdf(open(urdf).read(), end)
         robot = port.RobotSDFPort(chain, path_prefix=d, link_sdf_factory=port.cache_link_sdf_factory_port(0.02, 1.0))
@@ -680,7 +721,7 @@ def run_reference(args):
         others = {}
         for w in OTHER_WORKLOADS:
             try:
-                c, ms_w = _time_cpu_arm(cpu_arm(w), 2, 1, REFERENCE_OTHER_BUDGET_S)
+                c, ms_w = _time_cpu_arm(cpu_arm(w), args.steps, args.warmup, REFERENCE_OTHER_BUDGET_S)
                 others[w] = {"value": c["value"], "unit": UNIT, "ms_per_step": ms_w, "cpu_baseline": c}
             except Exception as e:      # never lose the headline to a secondary arm
                 others[w] = {"error": repr(e)[:200]}
@@ -699,9 +740,10 @@ def sum_over_ranks(x, world):
     return x
 
 
-def timed_steps(step, steps, warmup, world, sampler=None):
+def timed_steps(step, steps, warmup, world, sampler=None, last=None):
     """`warmup` untimed steps, then exactly `steps` steps bracketed by barrier + synchronize on both sides, timed with
-    CUDA events on the launch stream; returns (max-over-ranks ms for all steps, this rank's ms, host issue us/step)."""
+    CUDA events on the launch stream; returns (max-over-ranks ms for all steps, this rank's ms, host issue us/step).
+    `last`, if given, receives the result of the last timed step once the timing has ended."""
     out = None
     for i in range(warmup):             # same ownership pattern as the timed loop (the previous result stays alive
         out = step(i)                   # while the next one is allocated), so the allocator is in steady state
@@ -720,6 +762,8 @@ def timed_steps(step, steps, warmup, world, sampler=None):
         sampler.sample_now()            # the GPU is still executing the queued timed steps here
     barrier(world)
     mine = t_begin.elapsed_time(t_end)
+    if last is not None:
+        last(out)
     del out
     return max_over_ranks(mine, world), mine, issue_us
 
@@ -807,11 +851,11 @@ def cpu_baseline_of(name, wl=None, seconds=6.0):
     return {"value": done / dt, "unit": UNIT, "cores": cpu_threads, "kind": "port", "sample": sample}
 
 
-def run_workload(name, rank, world, steps, warmup, with_e2e, with_cpu, sampler=None, full_affinity=None):
+def run_workload(name, rank, world, steps, warmup, with_e2e, with_cpu, sampler=None, full_affinity=None, last=None):
     """One non-headline workload: device-resident value, independent kernel time + roofline, e2e, CPU baseline."""
     wl = make_workload(name, rank, world)
     torch.cuda.synchronize()
-    total_ms, _, issue_us = timed_steps(wl.step, steps, warmup, world, sampler)
+    total_ms, _, issue_us = timed_steps(wl.step, steps, warmup, world, sampler, last)
     units_all = max_over_ranks(float(wl.units), world) * world if name in WEAK_SCALED \
         else sum_over_ranks(float(wl.units), world)
     res = {"value": units_all * steps / (total_ms * 1e-3), "unit": UNIT, "ms_per_step": total_ms / steps,
@@ -819,7 +863,7 @@ def run_workload(name, rank, world, steps, warmup, with_e2e, with_cpu, sampler=N
            "gpu_launches": wl.launches_per_step * steps, "host_issue_us_per_step": issue_us}
     res["roofline"] = roofline_of(wl, kernel_time_ms(wl.step))
     if with_e2e:
-        res["e2e"] = e2e_arm(wl, units_all, world, max(3, min(steps, 10)))
+        res["e2e"] = e2e_arm(wl, units_all, world, steps)
     if with_cpu:
         with all_host_cpus(full_affinity):
             res["cpu_baseline"] = cpu_baseline_of(name, wl)
@@ -839,7 +883,13 @@ def main():
     ap.add_argument("--no-workloads", action="store_true", help="default run: headline only")
     ap.add_argument("--mode", default=None, choices=[None, "none", "nccl", "peer", "mc", "dma"],
                     help="C4 at N>1: force the re-assembly method of the headline instead of picking the faster one")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the results of the native path")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -855,11 +905,12 @@ def main():
     barrier(world)
     sampler = ClockSampler(local)
     with_cpu = rank == 0 and world == 1 and not args.no_cpu_baseline
+    dump = (lambda out: dump_outputs(out, args.dump_outputs)) if args.dump_outputs and rank == 0 else None
 
     if args.workload != "default" and args.workload not in ("c4", "c4readme"):
         # ---- single-workload mode (tuning / profiling scripts) ----
         wl, res = run_workload(args.workload, rank, world, args.steps, args.warmup, not args.no_e2e, with_cpu,
-                               sampler, full_affinity)
+                               sampler, full_affinity, dump)
         clocks = sampler.stop()
         if rank == 0:
             line = {"metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
@@ -875,39 +926,38 @@ def main():
     wl = make_workload("c4" if args.workload == "default" else args.workload, rank, world)
     torch.cuda.synchronize()
     units_all = sum_over_ranks(float(wl.units), world)
-    sub_steps = max(5, min(args.steps, 20))
     reassembly = None
     if world > 1:
         reassembly = {}
         wl.set_mode("none")
-        ms, _, _ = timed_steps(wl.step, sub_steps, args.warmup, world)
-        reassembly["no_reassembly"] = {"ms_per_step": ms / sub_steps, "value": units_all * sub_steps / (ms * 1e-3)}
+        ms, _, _ = timed_steps(wl.step, args.steps, args.warmup, world)
+        reassembly["no_reassembly"] = {"ms_per_step": ms / args.steps, "value": units_all * args.steps / (ms * 1e-3)}
         wl.set_mode("nccl")
-        ms, _, _ = timed_steps(wl.step, sub_steps, args.warmup, world)
-        reassembly["nccl_all_gather"] = {"ms_per_step": ms / sub_steps, "value": units_all * sub_steps / (ms * 1e-3)}
+        ms, _, _ = timed_steps(wl.step, args.steps, args.warmup, world)
+        reassembly["nccl_all_gather"] = {"ms_per_step": ms / args.steps, "value": units_all * args.steps / (ms * 1e-3)}
         err = wl.enable_peer()
         if err is None:
             wl.set_mode("peer")
-            ms, _, _ = timed_steps(wl.step, sub_steps, args.warmup, world)
+            ms, _, _ = timed_steps(wl.step, args.steps, args.warmup, world)
             remote = 16.0 * wl.units * (world - 1)          # bytes this rank pushes to its peers per step
-            reassembly["peer_stores"] = {"ms_per_step": ms / sub_steps, "value": units_all * sub_steps / (ms * 1e-3),
-                                         "nvlink_out_GBps_per_rank": remote / (ms / sub_steps * 1e-3) / 1e9,
+            reassembly["peer_stores"] = {"ms_per_step": ms / args.steps, "value": units_all * args.steps / (ms * 1e-3),
+                                         "nvlink_out_GBps_per_rank": remote / (ms / args.steps * 1e-3) / 1e9,
                                          "nvlink_in_bytes_per_rank": remote, "buffers": wl.peer.backend}
             slab = wl.end - wl.begin
             for pieces in (1, 2, 4):         # copy-engine pushes: the slab at once, or in pieces that overlap the kernel
                 wl.peer.dma_chunk_cfgs = 0 if pieces == 1 else max(1, -(-slab // pieces))
                 wl.set_mode("dma")
-                ms, _, _ = timed_steps(wl.step, sub_steps, args.warmup, world)
+                ms, _, _ = timed_steps(wl.step, args.steps, args.warmup, world)
                 reassembly[f"dma_push_{pieces}"] = {
-                    "ms_per_step": ms / sub_steps, "value": units_all * sub_steps / (ms * 1e-3),
+                    "ms_per_step": ms / args.steps, "value": units_all * args.steps / (ms * 1e-3),
                     "chunk_cfgs": wl.peer.dma_chunk_cfgs or slab,
-                    "nvlink_ingest_GBps_per_rank": 16.0 * (units_all - wl.units) / (ms / sub_steps * 1e-3) / 1e9}
+                    "nvlink_ingest_GBps_per_rank": 16.0 * (units_all - wl.units) / (ms / args.steps * 1e-3) / 1e9}
             if wl.peer.multicast:
                 wl.set_mode("mc")
-                ms, _, _ = timed_steps(wl.step, sub_steps, args.warmup, world)
-                reassembly["multicast_stores"] = {"ms_per_step": ms / sub_steps,
-                                                  "value": units_all * sub_steps / (ms * 1e-3),
-                                                  "nvlink_out_GBps_per_rank": 16.0 * wl.units / (ms / sub_steps * 1e-3) / 1e9}
+                ms, _, _ = timed_steps(wl.step, args.steps, args.warmup, world)
+                reassembly["multicast_stores"] = {"ms_per_step": ms / args.steps,
+                                                  "value": units_all * args.steps / (ms * 1e-3),
+                                                  "nvlink_out_GBps_per_rank": 16.0 * wl.units / (ms / args.steps * 1e-3) / 1e9}
             else:
                 reassembly["multicast_stores"] = {"unavailable": wl.peer.backend_note or
                                                   f"no multicast mapping (buffers: {wl.peer.backend})"}
@@ -944,18 +994,18 @@ def main():
         reassembly["chosen"] = chosen
         wl.set_mode(chosen)
 
-    total_ms, _, issue_us = timed_steps(wl.step, args.steps, args.warmup, world, sampler)
+    total_ms, _, issue_us = timed_steps(wl.step, args.steps, args.warmup, world, sampler, dump)
     clocks = sampler.stop()
     value = units_all * args.steps / (total_ms * 1e-3)
     kernel_ms = kernel_time_ms(wl.step)
     roofline = roofline_of(wl, kernel_ms)
     # FK + query through the public API (set_joint_configuration is part of every control-loop iteration)
-    rq_ms, _, _ = timed_steps(wl.step_reconfigure, sub_steps, 3, world)
-    reconfigure = {"ms_per_step": rq_ms / sub_steps, "value": units_all * sub_steps / (rq_ms * 1e-3),
+    rq_ms, _, _ = timed_steps(wl.step_reconfigure, args.steps, 3, world)
+    reconfigure = {"ms_per_step": rq_ms / args.steps, "value": units_all * args.steps / (rq_ms * 1e-3),
                    "what": "RobotSDF.set_joint_configuration(q[200,7]) + the headline step, device-resident inputs"}
     e2e = None
     if not args.no_e2e:
-        e2e = e2e_arm(wl, units_all, world, max(3, min(args.steps, 10)))
+        e2e = e2e_arm(wl, units_all, world, args.steps)
         wl.restore()
     cpu = None
     if with_cpu:
@@ -973,7 +1023,7 @@ def main():
         others = {}
         for name in OTHER_WORKLOADS:
             try:
-                w, res = run_workload(name, rank, world, min(args.steps, 30), args.warmup, not args.no_e2e,
+                w, res = run_workload(name, rank, world, args.steps, args.warmup, not args.no_e2e,
                                       with_cpu, None, full_affinity)
                 others[name] = res
                 del w

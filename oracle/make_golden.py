@@ -54,6 +54,22 @@ def make_meshes():
     print("meshes.npz:", {k: v.shape for k, v in out.items()})
 
 
+def save_split(name, arrays):
+    """<name>.npz, with the voxel tables in <name>.tables.npz and the fp32-range variant in <name>.f32range.npz so that
+    every fixture file stays below 1 MB (tests/helpers.py golden() merges the parts)."""
+    parts = {"": {}, ".tables": {}, ".f32range": {}}
+    for k, v in arrays.items():
+        if k.startswith("table_") and k != "table_shape":
+            parts[".tables"][k] = v
+        elif k.endswith("_f32range"):
+            parts[".f32range"][k] = v
+        else:
+            parts[""][k] = v
+    for suffix, part in parts.items():
+        if part:
+            np.savez_compressed(os.path.join(GOLD, f"{name}{suffix}.npz"), **part)
+
+
 def ray_noise_for(n, seed):
     """Seeds numpy's global generator so that the reference's np.random.randn(*shape) draw (sdf.py:149) is
     reproducible; returns nothing -- the port re-seeds identically."""
@@ -130,7 +146,7 @@ def make_reference_vectors():
                        inbound_f32range=c32.voxels.get_valid_values(q).numpy(),
                        table_val_f32range=c32.voxels.raw_data.numpy(), table_grad_f32range=c32.voxels_grad.numpy(),
                        ranges_f32range=np.array(c32.ranges))
-        np.savez_compressed(os.path.join(GOLD, f"ref_cachedsdf_{name}.npz"), **out)
+        save_split(f"ref_cachedsdf_{name}", out)
         print(name, "cachedsdf: table", tuple(c.voxels.shape), "inbound fraction", float(inb.float().mean()))
 
     # ---- ComposedSDF: 3 cached probes + sphere, plain and config-batched (sdf.py:332-433) ----
@@ -200,6 +216,30 @@ def make_reference_vectors():
         np.savez_compressed(os.path.join(GOLD, f"ref_chamfer_{name}.npz"), pts_world=pts_world.numpy(),
                             w2o=w2o.numpy(), err0=err0.numpy(), w2o_p=w2o_p.numpy(), err1=err1.numpy())
         print(name, "chamfer: err0 max", float(err0.max()), "err1 mean", float(err1.mean()))
+
+
+def make_robot_build_vectors():
+    """The single-link robot of tests/test_model_to_sdf.py:263-290 with the link table built by the reference itself
+    (resolution 0.008): pins the port's table build + RobotSDF query (tests/test_oracle_pinning.py)."""
+    pv = import_reference()
+    import pytorch_kinematics as pk
+    tmp = "/tmp/pvb_golden_cache"
+    os.makedirs(tmp, exist_ok=True)
+    urdf = open(os.path.join(REF, "tests", "offset_wrench.urdf")).read()
+    chain = pk.build_serial_chain_from_urdf(urdf, "offset_wrench")
+    np.random.seed(1)
+    rs = pv.RobotSDF(chain, path_prefix=os.path.join(REF, "tests"),
+                     link_sdf_cls=pv.cache_link_sdf_factory(resolution=0.008, padding=0.05,
+                                                            cache_path=os.path.join(tmp, "sdf_wrench_008.pkl"),
+                                                            clean_cache=True))
+    th = torch.tensor([[0.01, -0.02, 0.0, 0.3, -0.2, 0.5], [0.0, 0.0, 0.0, 0.0, 0.0, 0.0]])
+    rs.set_joint_configuration(th)
+    q = (torch.rand(500, 3, generator=torch.Generator().manual_seed(5)) - 0.5) * 0.4
+    v, g = rs(q)
+    bb = rs.surface_bounding_box(padding=0.01)
+    np.savez_compressed(os.path.join(GOLD, "ref_robot_wrench_built.npz"), th=th.numpy(), q=q.numpy(), val=v.numpy(),
+                        grad=g.numpy(), bbox=bb.numpy())
+    print("robot (reference-built table):", v.shape, bb.shape)
 
 
 def make_voxel_vectors():
@@ -273,7 +313,10 @@ if __name__ == "__main__":
     os.makedirs(GOLD, exist_ok=True)
     if len(sys.argv) > 1 and sys.argv[1] == "voxel":
         make_voxel_vectors()
+    elif len(sys.argv) > 1 and sys.argv[1] == "robot_build":
+        make_robot_build_vectors()
     else:
         make_meshes()
         make_reference_vectors()
+        make_robot_build_vectors()
         make_voxel_vectors()

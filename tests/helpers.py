@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests (test infrastructure; may use oracle/)."""
+import glob
 import os
 
 import numpy as np
@@ -11,8 +12,14 @@ GOLDEN = workloads.GOLDEN
 
 
 def golden(name):
-    with np.load(os.path.join(GOLDEN, name + ".npz")) as z:
-        return {k: z[k] for k in z.files}
+    """Arrays of tests/golden/<name>.npz merged with those of its parts <name>.<part>.npz (a fixture is split into
+    parts to keep every file small)."""
+    out = {}
+    for path in [os.path.join(GOLDEN, name + ".npz")] + sorted(glob.glob(os.path.join(GOLDEN, name + ".*.npz"))):
+        with np.load(path) as z:
+            assert not set(z.files) & set(out), path
+            out.update({k: z[k] for k in z.files})
+    return out
 
 
 def port_mesh(name):

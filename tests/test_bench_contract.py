@@ -4,6 +4,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ENV = dict(os.environ, PVB_BENCH_REF_BUDGET_S="3")      # the driver's run uses the full budget; the CPU tier a short one
 
@@ -46,6 +48,35 @@ def test_reference_arm_other_ranks_exit_quietly():
                           "--warmup", "0", "--gpus", "2"], stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True,
                          timeout=600, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_dump_outputs_sample(tmp_path):
+    """--dump-outputs: a result over the byte budget is sampled along the point axis at the same indices in every run;
+    one within it is written whole; float32 on disk."""
+    sys.path.insert(0, ROOT)
+    import bench
+    import torch
+    g = torch.Generator().manual_seed(1)
+    val = torch.randn(200, 100_000, generator=g)
+    grad = torch.randn(200, 100_000, 3, generator=g)
+    for d in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs((val, grad), str(d))
+    v, gr = np.load(tmp_path / "a" / "value.npy"), np.load(tmp_path / "a" / "gradient.npy")
+    assert v.dtype == np.float32 and gr.dtype == np.float32
+    assert v.nbytes + gr.nbytes <= bench.DUMP_MAX_BYTES <= 64 << 20
+    k = v.shape[1]
+    assert v.shape == (200, k) and gr.shape == (200, k, 3) and k > 10_000
+    assert np.array_equal(np.load(tmp_path / "b" / "value.npy"), v)
+    assert np.array_equal(np.load(tmp_path / "b" / "gradient.npy"), gr)
+    # the sample is one set of point columns: each column of the dump is a column of the result, in index order
+    cols = [int(np.flatnonzero((val[0].numpy() == v[0, j]))[0]) for j in (0, k // 2, k - 1)]
+    assert cols == sorted(cols)
+    for j, c in zip((0, k // 2, k - 1), cols):
+        assert np.array_equal(v[:, j], val[:, c].numpy()) and np.array_equal(gr[:, j], grad[:, c].numpy())
+    small = torch.arange(12, dtype=torch.float64)
+    bench.dump_outputs(small, str(tmp_path / "c"))
+    assert np.array_equal(np.load(tmp_path / "c" / "value.npy"), small.numpy())
+    assert not (tmp_path / "c" / "gradient.npy").exists()
 
 
 def test_committed_ncu_side_files_cover_every_workload():

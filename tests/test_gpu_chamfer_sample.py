@@ -27,7 +27,7 @@ def test_chamfer_vs_reference_golden(name):
         pv.batch_chamfer_dist(torch.from_numpy(z["w2o"]).cuda(), pts)
 
 
-def test_chamfer_reference_invariants():
+def test_chamfer_reference_invariants(tmp_path):
     """tests/test_chamfer.py:40-66: mesh chamfer < point-cloud chamfer and within 5 % of it."""
     import pytorch_volumetric_b200 as pv
     torch.manual_seed(3)
@@ -46,7 +46,7 @@ def test_chamfer_reference_invariants():
     assert torch.all(manual - err < 0.05 * manual)
     # obj_sdf route (chamfer.py:84-85) on a CachedSDF of the same object
     c = pv.CachedSDF("probe", 0.001, obj.bounding_box(padding=0.3), pv.MeshSDF(obj), device="cuda",
-                     cache_path="/tmp/pvb_test_chamfer_cache.pkl", clean_cache=True)
+                     cache_path=str(tmp_path / "cache.pkl"), clean_cache=True)
     err_c = pv.batch_chamfer_dist(pert.inverse().get_matrix(), pts_world, obj_sdf=c, scale=1) * N
     assert torch.all((err_c - err).abs() < 0.1 * err + 1e-3)
 

@@ -1,19 +1,12 @@
-"""CPU: pins oracle/port.py (the restatement of the reference's own code) against
- (a) the golden vectors written by the UNMODIFIED reference source over oracle/shims (oracle/make_golden.py), and
- (b) when /root/reference is present (build container), a live run of that source.
-The third-party layer under both is the same restatement, so agreement here is bit-exact."""
-import os
-import sys
-
+"""CPU: pins oracle/port.py (the restatement of the reference's own code) against the golden vectors written by the
+UNMODIFIED reference source over oracle/shims (oracle/make_golden.py).  The third-party layer under both is the same
+restatement, so agreement here is bit-exact."""
 import numpy as np
 import pytest
 import torch
 
-import workloads
 from helpers import golden, port_mesh
 from oracle import port, tp_pytorch_kinematics as opk
-
-HAVE_REF = os.path.isdir("/root/reference/src/pytorch_volumetric")
 
 
 @pytest.mark.parametrize("name", ["probe", "wrench", "drill"])
@@ -115,50 +108,27 @@ def test_port_chamfer_equals_reference_golden(oracle_lib):
         port.batch_chamfer_dist_port(torch.from_numpy(z["w2o_p"]), torch.from_numpy(z["pts_world"]))
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference only exists in the build container")
 def test_port_equals_live_reference_source(tmp_path, oracle_lib):
-    """Imports the real reference package (its third-party imports resolved by oracle/shims) and runs the single
-    link robot of tests/test_model_to_sdf.py:263-290 through both the reference and the port."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    saved = list(sys.path)
-    try:
-        sys.path.insert(0, os.path.join(root, "oracle", "shims"))
-        sys.path.insert(0, "/root/reference/src")
-        import pytorch_volumetric as pv
-        import pytorch_kinematics as pk
-        assert pv.__file__.startswith("/root/reference")
-        urdf = open("/root/reference/tests/offset_wrench.urdf").read()
-        chain = pk.build_serial_chain_from_urdf(urdf, "offset_wrench")
-        np.random.seed(1)
-        rs = pv.RobotSDF(chain, path_prefix="/root/reference/tests",
-                         link_sdf_cls=pv.cache_link_sdf_factory(resolution=0.008, padding=0.05,
-                                                                cache_path=str(tmp_path / "a.pkl")))
-        th = torch.tensor([[0.01, -0.02, 0.0, 0.3, -0.2, 0.5], [0.0, 0.0, 0.0, 0.0, 0.0, 0.0]])
-        rs.set_joint_configuration(th)
-        q = (torch.rand(500, 3, generator=torch.Generator().manual_seed(5)) - 0.5) * 0.4
-        v_ref, g_ref = rs(q)
-        bb_ref = rs.surface_bounding_box(padding=0.01)
-
-        chain2 = opk.build_serial_chain_from_urdf(urdf, "offset_wrench")
-        np.random.seed(1)
-        rp = port.RobotSDFPort(chain2, path_prefix="/root/reference/tests",
-                               link_sdf_factory=port.cache_link_sdf_factory_port(resolution=0.008, padding=0.05))
-        rp.set_joint_configuration(th)
-        v, g = rp(q)
-        assert torch.equal(v, v_ref) and torch.equal(g, g_ref)
-        assert torch.equal(rp.surface_bounding_box(padding=0.01), bb_ref)
-    finally:
-        sys.path[:] = saved
-        for m in [m for m in sys.modules if m.split(".")[0] in ("pytorch_volumetric", "open3d", "multidim_indexing",
-                                                                "pytorch_kinematics", "arm_pytorch_utilities",
-                                                                "matplotlib")]:
-            del sys.modules[m]
+    """The single link robot of tests/test_model_to_sdf.py:263-290 with the link table built by the port itself:
+    values, gradients and bounding box equal what the unmodified reference source computed for the same inputs
+    with its own table build (oracle/make_golden.py: ref_robot_wrench_built)."""
+    from test_gpu_composed import write_wrench_urdf
+    z = golden("ref_robot_wrench_built")
+    urdf = write_wrench_urdf(str(tmp_path))
+    chain = opk.build_serial_chain_from_urdf(open(urdf).read(), "offset_wrench")
+    np.random.seed(1)
+    rp = port.RobotSDFPort(chain, path_prefix=str(tmp_path),
+                           link_sdf_factory=port.cache_link_sdf_factory_port(resolution=0.008, padding=0.05))
+    rp.set_joint_configuration(torch.from_numpy(z["th"]))
+    v, g = rp(torch.from_numpy(z["q"]))
+    assert np.array_equal(v.numpy(), z["val"]) and np.array_equal(g.numpy(), z["grad"])
+    assert np.array_equal(rp.surface_bounding_box(padding=0.01).numpy(), z["bbox"])
 
 
 def test_port_robot_equals_reference_golden(tmp_path, oracle_lib):
     """RobotSDFPort on the procedural twin of the reference's tests/offset_wrench.urdf reproduces the vectors the
     unmodified reference produced (oracle/make_golden.py: ref_robot_wrench) -- FK + offset composition bit-exact,
-    values / gradients bit-exact on the reference-built link table.  Runs without /root/reference."""
+    values / gradients bit-exact on the reference-built link table."""
     from oracle import tp_pytorch_kinematics as opk
     from test_gpu_composed import write_wrench_urdf
     z = golden("ref_robot_wrench")
